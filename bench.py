@@ -2,11 +2,14 @@
 """PPO-update throughput benchmark (BASELINE.json metric: PPO-update samples/sec on
 64x64x4 depth + proprio rollouts).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--model loco|nature] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--model loco|nature] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one PPO.update_per_epoch() over a synthetic rollout of T x E transitions:
 GAE scan + opt_epochs x (T*E/B) minibatch updates (critic fwd/bwd/clip/Adam, actor fwd/bwd +
-frozen-target fwd/clip/Adam) = opt_epochs*T*E sample-updates.
+frozen-target fwd/clip/Adam) = opt_epochs*T*E sample-updates.  Every step, warm-up and timed, starts from the
+same network and optimiser state: in training each update sees a fresh rollout drawn near the current policy,
+while updates chained over this one fixed rollout drive the policy ever further from its actions until the
+importance ratios overflow (after ~20 steps, in the exact fp32 tier as well).
   value : rollout already resident in HBM when the timed region starts (CUDA events, max over
           ranks);
   e2e   : the same step through the public call PPO.update_per_epoch() with the rollout in
@@ -72,7 +75,13 @@ def parse():
   ap.add_argument("--sweep-timeout", type=int, default=300)
   ap.add_argument("--sweep-envs", type=int, default=8, help="env columns of the sweep's rollout (8 = BASELINE configs[4])")
   ap.add_argument("--no-roofline", action="store_true")
-  return ap.parse_args()
+  ap.add_argument("--dump-outputs", metavar="DIR",
+                  help="write what the last timed step computed (per-minibatch statistics, parameters after the step, "
+                       "advantages and returns) to DIR/<name>.npy, to compare two builds output for output")
+  args = ap.parse_args()
+  if args.dump_outputs and args.steps < 1:
+    ap.error("--dump-outputs needs at least one timed step")
+  return args
 
 
 def peaks():
@@ -356,8 +365,14 @@ def main():
   np.random.seed(0)
   eng.load_rollout(buf)
   last = buf.last_sample(["next_obs", "terminals"])
+  start = [t.clone() for t in training_state(eng)]
+
+  def restart():
+    for t, t0 in zip(training_state(eng), start):
+      t.copy_(t0)
 
   def resident_step(epoch):
+    restart()
     agent.current_epoch = epoch
     eng.compute_advantages(last["next_obs"], last["terminals"], agent.discount, agent.tau, True, True)
     agent._schedule()
@@ -377,10 +392,12 @@ def main():
   t_w0 = time.perf_counter()
   ev0.record()
   for k in range(args.steps):
-    resident_step(args.warmup + k)
+    infos = resident_step(args.warmup + k)
   ev1.record()
   barrier()
   t_w1 = time.perf_counter()
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, infos, pf, vf, eng._roll)
   ms = max_over_ranks(ev0.elapsed_time(ev1))
   launches = eng.ops.launches - launches0
   clocks = sampler.stop((t_w0, t_w1)) if rank == 0 else None
@@ -388,12 +405,14 @@ def main():
 
   # ---- end-to-end step through the public API with HOST buffers
   for w in range(2):
+    restart()
     agent.current_epoch = w
     agent.update_per_epoch()
   barrier()
   t0 = time.perf_counter()
   ev0.record()
   for k in range(args.steps):
+    restart()
     agent.current_epoch = 10 + k
     agent.update_per_epoch()
   ev1.record()
@@ -475,6 +494,38 @@ def main():
   sys.stdout.flush()
   if world > 1:
     os._exit(0)
+
+
+def training_state(eng):
+  """what one step changes: the parameters of both networks (one flat bucket), the Adam moments and step counts"""
+  return [eng.bucket.flat, eng.m_pf, eng.v_pf, eng.m_vf, eng.v_vf, eng.hyper_pf, eng.hyper_vf]
+
+
+DUMP_MAX_ELEMS = 1 << 20          # per array: larger arrays are stored as a fixed, seeded sample
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(d, infos, pf, vf, roll):
+  """What a caller of the timed step receives, after its last call: the logged statistics of every minibatch
+  (float64, one row per minibatch), the parameters of both networks (float32) and the step's advantages and returns
+  (float32, [T*E]).  An array of more than DUMP_MAX_ELEMS elements is replaced by the values at
+  sorted(default_rng(0).choice(n, DUMP_MAX_ELEMS, replace=False)) of its flattened form."""
+  from vision4leg_b200._lib import INFO_KEYS
+  out = {"info.%s" % k.replace("/", "_"): np.array([float(i[k]) for i in infos], np.float64) for k in INFO_KEYS}
+  for name, net in (("pf", pf), ("vf", vf)):
+    for k, v in net.state_dict().items():
+      out["%s.%s" % (name, k)] = v.detach().float().cpu().numpy()
+  out["gae.advs"] = roll["advs"].detach().float().cpu().numpy().reshape(-1)
+  out["gae.returns"] = roll["rets"].detach().float().cpu().numpy().reshape(-1)
+  for k, a in out.items():
+    if a.size > DUMP_MAX_ELEMS:
+      out[k] = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+  total = sum(a.nbytes for a in out.values())
+  if total > DUMP_MAX_BYTES:
+    raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte bound" % (total, DUMP_MAX_BYTES))
+  os.makedirs(d, exist_ok=True)
+  for k, a in out.items():
+    np.save(os.path.join(d, k + ".npy"), a)
 
 
 # -------------------------------------------------------------------------------------------------

@@ -3,13 +3,12 @@ reference (viewers, TensorRT export): `model_{pf,vf}_{epoch}.pth` = plain state_
 `_obs_normalizer_{epoch}.pkl` = a pickled torchrl.env.base_wrapper.Normalizer (reference rl_algo.py:84-95).
 
 The fixture tests/golden/obs_normalizer_ref.pkl was written by the live reference (oracle/make_golden_obs.py).
-Two tests load OUR files into the LIVE reference in a subprocess; they need /root/reference and are skipped
-where it does not exist (the GPU box)."""
+tests/golden/checkpoint_wire.npz records what the live reference did with OUR files (oracle/make_golden_wire.py):
+the bytes of our normaliser pickle it loaded and what it computed from them, the key order / shapes / dtypes of its
+modules after a strict load of our state_dicts and their forward outputs."""
 import io
 import os
 import pickle
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -18,9 +17,7 @@ import torch
 from tests import _golden as g
 from vision4leg_b200 import obs_pipeline as op
 
-REF = os.environ.get("V4L_REFERENCE_ROOT", "/root/reference")
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "torchrl")), reason="no reference checkout here")
+WIRE = os.path.join(g.GOLDEN_DIR, "checkpoint_wire.npz")
 
 
 def _globals(stream):
@@ -76,65 +73,53 @@ def test_our_pickle_names_only_the_reference_class():
                                                      st["should_estimate"])) == raw
 
 
-def _run_in_reference(code, *argv):
-  env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1", PYTHONPATH=ROOT)
-  r = subprocess.run([sys.executable, "-c", code] + list(argv), env=env, capture_output=True, text=True, timeout=300)
-  assert r.returncode == 0, r.stdout + r.stderr
-  return r.stdout
-
-
-@needs_reference
-def test_live_reference_loads_our_normalizer_pickle(tmp_path):
+def normalizer_case():
+  """(bytes of the `_obs_normalizer_7.pkl` we write for a device normaliser with these statistics, filter input)"""
   rng = np.random.RandomState(3)
   mean, var = rng.randn(37), rng.rand(37) + 0.5
-  path = str(tmp_path / "_obs_normalizer_7.pkl")
-  with open(path, "wb") as f:
-    pickle.dump(_DeviceStandIn(dict(shape=(37,), _mean=mean, _var=var, _count=123.0001, clip=10., should_estimate=True)), f)
-  x = rng.randn(4, 37)
-  np.save(str(tmp_path / "x.npy"), x)
-  out = _run_in_reference("""
-import sys, pickle, types, importlib.util, numpy as np
-gym = types.ModuleType("gym")
-for n in ("Wrapper", "RewardWrapper", "ObservationWrapper"):
-  setattr(gym, n, type(n, (), {}))
-sys.modules["gym"] = gym
-spec = importlib.util.spec_from_file_location("torchrl.env.base_wrapper", sys.argv[1] + "/torchrl/env/base_wrapper.py")
-mod = importlib.util.module_from_spec(spec); sys.modules["torchrl.env.base_wrapper"] = mod; spec.loader.exec_module(mod)
-nz = pickle.load(open(sys.argv[2], "rb"))
-assert type(nz) is mod.Normalizer, type(nz)
-np.save(sys.argv[3], nz.filt(np.load(sys.argv[4])))
-print(nz._count)
-""", REF, path, str(tmp_path / "y.npy"), str(tmp_path / "x.npy"))
-  assert float(out.strip()) == 123.0001
-  want = np.clip((x - mean) / (np.sqrt(var) + 1e-4), -10, 10)
-  assert np.array_equal(np.load(str(tmp_path / "y.npy")), want)
+  raw = pickle.dumps(_DeviceStandIn(dict(shape=(37,), _mean=mean, _var=var, _count=123.0001, clip=10.,
+                                         should_estimate=True)))
+  return raw, rng.randn(4, 37)
 
 
-@needs_reference
-@pytest.mark.parametrize("family", ["loco", "mlp"])
-def test_live_reference_loads_our_state_dicts(tmp_path, family):
-  """model_{pf,vf}_{epoch}.pth written the way RLAlgo.snapshot writes them load into the reference's own modules
-  with strict=True and reproduce the reference's forward fixture"""
+def save_state_dicts(family, d):
+  """model_{pf,vf}_3.pth the way RLAlgo.snapshot writes them, for the family's fixture weights"""
   from benchutil.harness import build_nets, load_np_sd
   S, A = g.FAMILIES[family]
   pf, vf = build_nets(family, S, A)
   pf_np, vf_np = g.family_weights(family)
   load_np_sd(pf, pf_np); load_np_sd(vf, vf_np)
   for name, net in (("pf", pf), ("vf", vf)):
-    torch.save({k: v.detach().clone() for k, v in net.state_dict().items()}, str(tmp_path / ("model_%s_3.pth" % name)))
-  _run_in_reference("""
-import sys, numpy as np, torch
-from oracle import make_golden as mg
-from tests import _golden as g
-family, d = sys.argv[1], sys.argv[2]
-obs, acts = g.fwd_inputs(family)
-G = g.load(family)
-networks, policies, PPO, Buffer, Box = mg.import_reference()
-S, A = mg.FAMILIES[family]
-pf, vf = mg.build_reference_nets(networks, policies, family, S, A)
-pf.load_state_dict(torch.load(d + "/model_pf_3.pth", map_location="cpu"), strict=True)
-vf.load_state_dict(torch.load(d + "/model_vf_3.pth", map_location="cpu"), strict=True)
-with torch.no_grad():
-  assert np.allclose(vf(torch.tensor(obs)).numpy(), G["fwd/value"], rtol=1e-5, atol=1e-6)
-  assert np.allclose(pf.update(torch.tensor(obs), torch.tensor(acts))["mean"].numpy(), G["fwd/mean"], rtol=1e-5, atol=1e-6)
-""", family, str(tmp_path))
+    torch.save({k: v.detach().clone() for k, v in net.state_dict().items()}, os.path.join(d, "model_%s_3.pth" % name))
+  return pf_np, vf_np
+
+
+def test_live_reference_loads_our_normalizer_pickle():
+  """the reference unpickled these very bytes as its own Normalizer and filtered with the statistics they carry"""
+  W = np.load(WIRE)
+  raw, x = normalizer_case()
+  assert raw == W["norm/pickle"].tobytes()
+  rng = np.random.RandomState(3)
+  mean, var = rng.randn(37), rng.rand(37) + 0.5
+  assert float(W["norm/count"]) == 123.0001
+  want = np.clip((x - mean) / (np.sqrt(var) + 1e-4), -10, 10)
+  assert np.array_equal(W["norm/filt"], want)
+
+
+@pytest.mark.parametrize("family", ["loco", "mlp"])
+def test_live_reference_loads_our_state_dicts(tmp_path, family):
+  """model_{pf,vf}_{epoch}.pth written the way RLAlgo.snapshot writes them carry the reference's keys, in its order,
+  with its shapes and dtypes (what its strict load_state_dict took), holding the fixture weights under those keys; the
+  reference's modules loaded from them reproduce the reference's forward fixture"""
+  W = np.load(WIRE)
+  G = g.load(family)
+  weights = dict(zip(("pf", "vf"), save_state_dicts(family, str(tmp_path))))
+  for name in ("pf", "vf"):
+    sd = torch.load(str(tmp_path / ("model_%s_3.pth" % name)), map_location="cpu")
+    assert list(sd.keys()) == list(W["sd/%s/%s/keys" % (family, name)])
+    assert [",".join(map(str, v.shape)) for v in sd.values()] == list(W["sd/%s/%s/shapes" % (family, name)])
+    assert [str(v.dtype) for v in sd.values()] == list(W["sd/%s/%s/dtypes" % (family, name)])
+    for k, v in sd.items():
+      assert np.array_equal(v.numpy(), weights[name][k]), (name, k)
+  assert np.allclose(W["sd/%s/value" % family], G["fwd/value"], rtol=1e-5, atol=1e-6)
+  assert np.allclose(W["sd/%s/mean" % family], G["fwd/mean"], rtol=1e-5, atol=1e-6)

@@ -86,8 +86,6 @@ def test_autograd_through_modules_matches_oracle(family):
 @pytest.mark.parametrize("family", ALL)
 @pytest.mark.parametrize("clipped", [False, True])
 def test_one_update_matches_reference_golden(family, clipped):
-  if clipped and family in ("nature", "vit", "nvo"):
-    pytest.skip("no golden for this combination")
   G = g.load(family)
   pf, vf, S, A = _nets(family)
   agent, _ = make_ppo(pf, vf, None, A, 16, 16, 1, device=DEV, clipped_value_loss=clipped)

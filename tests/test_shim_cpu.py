@@ -1,15 +1,31 @@
 """The `torchrl/` drop-in shim (SURVEY 8(b): the boundary is "whatever starter/ppo_*.py import"): with this
 repo BEFORE a reference checkout on the path, the hot-path names resolve to vision4leg_b200 and everything
-else falls through to the reference.  Needs the reference checkout (skipped without it: the GPU box has none);
-`gym` is absent from this image, so the ten-line stub the oracle tooling uses stands in for it."""
+else falls through to the reference.  The checkout is a stand-in written by the test: a `torchrl/` tree with the
+reference's package layout, whose fall-through modules use the same kinds of imports (a relative import of a
+sibling the shim does not re-author, an absolute import of a shim-served module).  `gym` need not be installed:
+the ten-line stub the oracle tooling uses stands in for it."""
 import os
 import subprocess
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("V4L_REFERENCE_ROOT", "/root/reference")
+
+# path relative to the checkout -> source
+STAND_IN = {
+  "torchrl/__init__.py": "",
+  "torchrl/algo/__init__.py": "from .on_policy import *\nfrom .off_policy import *\n",
+  "torchrl/algo/on_policy/__init__.py": "from .a2c import A2C\nfrom .v_mpo import VMPO\n",
+  "torchrl/algo/on_policy/a2c.py": "class A2C:\n  pass\n",
+  "torchrl/algo/on_policy/v_mpo.py": "from .a2c import A2C\nimport torchrl.algo.utils as atu\n\n\n"
+                                     "class VMPO(A2C):\n  schedule = atu.update_linear_schedule\n",
+  "torchrl/algo/off_policy/__init__.py": "class SAC:\n  pass\n",
+  "torchrl/algo/utils.py": "",
+  "torchrl/networks/__init__.py": "",
+  "torchrl/policies/__init__.py": "",
+  "torchrl/replay_buffers/__init__.py": "",
+  "torchrl/replay_buffers/on_policy.py": "",
+}
+
 
 SCRIPT = r'''
 import sys, types
@@ -39,8 +55,11 @@ print("shim ok")
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "torchrl")), reason="no reference checkout")
-def test_torchrl_shim_resolution():
+def test_torchrl_shim_resolution(tmp_path):
+  for rel, src in STAND_IN.items():
+    (tmp_path / rel).parent.mkdir(parents=True, exist_ok=True)
+    (tmp_path / rel).write_text(src)
+  REF = str(tmp_path)
   env = dict(os.environ, PYTHONPATH=ROOT + os.pathsep + REF, V4L_REFERENCE_ROOT=REF, PYTHONDONTWRITEBYTECODE="1")
   out = subprocess.run([sys.executable, "-c", SCRIPT.replace("REF", repr(REF))], env=env, capture_output=True, text=True,
                        timeout=300)
